@@ -24,6 +24,12 @@ Keys:
              wrapper tiling on, cudnn.benchmark False and True - the north_star's ">= 4x" denominator (N = 1, c2/c3)
   parity_sharded      N > 1: rank 0 also runs the un-sharded clip and the gathered sharded result must be
              bit-identical (moments and reconstruction); the line carries the verdict
+  dumped     with --dump-outputs DIR: shape and stored element count of each array written to DIR
+
+--dump-outputs DIR writes what the last timed step computed (rank 0's share) as float32 .npy files: latent.npy, the
+latent z = encode(x).latent_dist.mode() that is decoded, and recon.npy, decode(z).sample.  An array of more than
+DUMP_MAX_ELEMS elements is stored as a fixed seeded sample of its flattened elements.  Weights and inputs are seeded,
+so runs with the same arguments on two builds can be compared array for array.  bench.py writes nothing into the tree.
 """
 from __future__ import annotations
 
@@ -38,7 +44,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; imports must not leave __pycache__ behind
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "video VAE encode+decode frames/sec at 17x576x1024"
@@ -74,7 +82,11 @@ def parse():
                     help="N > 1, batch-1 configs: 'frame' = clip sharded on the frame axis + halo exchange (default; c2/c3 grow the "
                          "clip with N), 'unit' = the FIXED clip resident on every rank, its (chunk x tile) work units dealt over "
                          "the ranks (strong scaling of a clip with fewer chunks than GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's latent and reconstruction to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     for k in ("frames", "height", "width", "dtype"):
         if getattr(args, k) is not None:
@@ -259,6 +271,31 @@ def run_reference(args, rank):
     print(json.dumps(line))
 
 
+# ------------------------------------------------------------------------------------------ output dump
+DUMP_MAX_ELEMS = 4 << 20   # per array: 16 MB of float32, so latent + reconstruction stay within 64 MB
+
+
+def dump_array(t, seed=0):
+    """`t` as a float32 numpy array, or, above DUMP_MAX_ELEMS elements, the flattened elements at DUMP_MAX_ELEMS sorted
+    positions drawn (with replacement) from a generator seeded with `seed`: the positions depend on the size alone."""
+    n = t.numel()
+    if n <= DUMP_MAX_ELEMS:
+        return t.float().cpu().numpy()
+    idx = torch.randint(0, n, (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return t.reshape(-1)[idx.to(t.device)].float().cpu().numpy()
+
+
+def dump_outputs(d, arrays):
+    """Write each named tensor to d/<name>.npy; returns {name: {"shape", "stored"}} for the JSON line."""
+    os.makedirs(d, exist_ok=True)
+    info = {}
+    for name, t in arrays.items():
+        a = dump_array(t)
+        np.save(os.path.join(d, name + ".npy"), a)
+        info[name] = {"shape": list(t.shape), "stored": int(a.size)}
+    return info
+
+
 # ------------------------------------------------------------------------------------------ GPU arms
 def build_model(cfg, dtype):
     from cvvae_b200 import CVVAEModel, CVVAESD3Model
@@ -338,11 +375,8 @@ def main():
     dtype = torch.float16 if args.dtype == "fp16" else torch.bfloat16
     zc = 4 if cfg["variant"] == "sd21" else 16
 
-    import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if world > 1:
-        dist.barrier()
+    from cvvae_b200 import _lib
+    _lib.load()   # the library __graft_entry__.build() made; bench.py compiles nothing and raises if it is missing
     model = build_model(cfg, dtype)
     ops = model._engine().ops
     if args.impl == "torch-cuda":
@@ -404,14 +438,16 @@ def main():
     x_dev = x_host.cuda()
 
     def step(x):
+        """One encode -> decode of this rank's share; returns (latent z, reconstruction)."""
         with torch.no_grad():
             if sharded is not None:
                 z = sharded.encode_local(x, total_chunks)[:, :zc].contiguous()
-                return sharded.decode_local(z, total_chunks)
+                return z, sharded.decode_local(z, total_chunks)
             if unit is not None:
-                return unit.decode(unit.encode(x)[:, :zc].contiguous())
+                z = unit.encode(x)[:, :zc].contiguous()
+                return z, unit.decode(z)
             z = net.tiled_encode(x)[:, :zc]
-            return net.tiled_decode(z)
+            return z, net.tiled_decode(z)
 
     def sync():
         torch.cuda.synchronize()
@@ -481,15 +517,19 @@ def main():
             sys.exit(1)
 
     for _ in range(max(args.warmup, 3)):
-        out = step(x_dev)
+        last = step(x_dev)
     sync()
+
+    def timed_step():
+        nonlocal last
+        last = step(x_dev)
 
     # ---- device-resident timing (+ per-conv CUDA events for the roofline)
     launches0 = ops.launch_count() if ops else 0
     sampler = ClockSampler(local) if rank == 0 else None
     if ops:
         ops.start_profile()
-    ms_total = timed(lambda: step(x_dev), args.steps)
+    ms_total = timed(timed_step, args.steps)
     ms_per_rank = getattr(timed, "per_rank", None)
     prof = ops.stop_profile() if ops else None
     clocks = sampler.stop() if sampler else None
@@ -497,13 +537,17 @@ def main():
     ms_step = ms_total / args.steps
     job_frames = B * total_frames
     value = job_frames / (ms_step * 1e-3)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, {"latent": last[0], "recon": last[1]})
+    out = last[1]
 
     # ---- end-to-end: pinned host clip -> H2D -> encode/decode -> D2H of the reconstruction, every step
     rec_host = torch.empty(out.shape, dtype=out.dtype).pin_memory()
 
     def e2e_step():
         xd = x_host.cuda(non_blocking=True)
-        r = step(xd)
+        r = step(xd)[1]
         rec_host.copy_(r, non_blocking=True)
 
     if args.impl == "ours":
@@ -573,6 +617,8 @@ def main():
         line["ms_per_step_per_rank"] = ms_per_rank
     if roof:
         line["roofline"] = roof
+    if dumped is not None:
+        line["dumped"] = dumped
     if args.impl == "ours" and world == 1:
         if not args.no_torch_baseline and args.config in ("c2", "c3"):
             ref = TorchCudaReference(cfg, dict(model.state_dict()))

@@ -9,7 +9,8 @@ The reference modules are imported verbatim from /root/reference through
 come from ``oracle.cvvae_oracle.make_state_dict`` (per-key seeded, so they can
 be regenerated anywhere) and are loaded into the reference with
 ``load_state_dict(strict=True)``; inputs from ``synthetic_video``.  Only the
-reference OUTPUTS are stored (fp32 .npz) plus a manifest describing each case.
+reference OUTPUTS are stored (fp32 .npz, large outputs as a fixed sample, see
+``tests/golden_data.py``) plus a manifest describing each case.
 """
 from __future__ import annotations
 
@@ -25,6 +26,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import golden_data  # noqa: E402
 import ref_shim  # noqa: E402
 
 ref_shim.install()
@@ -80,7 +82,7 @@ def build_reference(case):
 
 def main():
     manifest = {"weight_seed": WEIGHT_SEED, "input_seed": INPUT_SEED, "cases": []}
-    for case in CASES:
+    for i, case in enumerate(CASES):
         m, cfg, sd = build_reference(case)
         x = O.synthetic_video(case["shape"], INPUT_SEED)
         with torch.no_grad():
@@ -97,7 +99,7 @@ def main():
                 # 4-D latents regrouped with the model's own num_latent_frames (modeling_vae.py:308-309)
                 z4 = z.permute(0, 2, 1, 3, 4).reshape(-1, *z.shape[1:2], *z.shape[3:])
                 arrays["recon_4dlat"] = m.decode(z4).sample.numpy()
-        np.savez(os.path.join(HERE, case["name"] + ".npz"), **arrays)
+        np.savez(os.path.join(HERE, case["name"] + ".npz"), **golden_data.shrink(arrays, seed=i))
         shapes = {k: list(v) for k, v in O.param_shapes(cfg).items()}
         entry = dict(case)
         entry["shape"] = list(case["shape"])

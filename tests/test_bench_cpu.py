@@ -23,6 +23,23 @@ def test_workload_accounting_and_configs():
     assert bench.sample_shape(1)[3] == 192 and bench.sample_shape(23)[3] == 128 and bench.sample_shape(40)[3] == 96
 
 
+def test_dump_outputs_writes_float32_within_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    assert 2 * bench.DUMP_MAX_ELEMS * 4 <= 64 << 20                              # latent + recon as float32 <= 64 MB
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 1000)
+    small = torch.randn(2, 3, 4, dtype=torch.float16)
+    big = torch.arange(5000, dtype=torch.bfloat16)
+    info = bench.dump_outputs(str(tmp_path / "out"), {"latent": small, "recon": big})
+    assert info == {"latent": {"shape": [2, 3, 4], "stored": 24}, "recon": {"shape": [5000], "stored": 1000}}
+    a, b = np.load(tmp_path / "out" / "latent.npy"), np.load(tmp_path / "out" / "recon.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, small.float().numpy())   # small arrays whole and exact
+    assert b.dtype == np.float32 and b.shape == (1000,) and np.all(np.diff(b) >= 0) and set(b) <= set(big.float().numpy())
+    assert np.array_equal(b, bench.dump_array(big))                              # the sample is fixed
+
+
 def test_reference_arm_prints_one_contract_line():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                         "--height", "64", "--width", "64", "--frames", "5"], capture_output=True, text=True, timeout=900)
