@@ -50,7 +50,6 @@ struct ConvTcParams {
   int gn_groups, gn_cpg;
   int persist;  // persistent swap kernel: 256-position tiles, two TMEM stages, epilogue overlapped with the next tile
   int n_tiles;  // tiles of the whole launch (persistent kernel)
-  int swap;  // operands swapped: A = weights (M = 128 output channels), B = 256 positions (Cout == 128 layers)
   // persistent kernel, stride-1 layers: ONE slab per (kt, channel block) serves all KH x KW taps.  Tiles are 8 positions
   // wide (one 8-row swizzle group per image row), the slab keeps PW >= 8 + KW - 1 positions per row, and the UMMA
   // descriptor walks the image rows with SBO = PW * 128 B from a start address shifted by (kh * PW + kw) * 128 B.
@@ -422,20 +421,7 @@ __global__ void __launch_bounds__(kThreads, 1)
           first = false;
           const uint32_t b_lo0 = ((ptx::smem_u32(sB + static_cast<size_t>(slotB) * p.b_bytes) >> 4) & 0x3FFFu) | kDescLoFlags;
           const uint32_t a_lo1 = a_lo0 + static_cast<uint32_t>(khs) * tap_stride16;
-          if (p.swap) {
-            // D[channel lane][position column]: the weight tile is the M = 128 operand, 256 consecutive slab rows
-            // (two 128-position sub-tiles) the N operand -> 4 KB + 8 KB of operand reads per 128-cycle MMA instead of
-            // 4 KB + 4 KB per 64-cycle MMA, which is what bounds the N = 128 orientation
-            if (ptx::elect_one()) {
-              for (int a2 = 0; 2 * a2 < nacc_eff; ++a2) {
-                const uint32_t x_lo = a_lo1 + static_cast<uint32_t>(2 * a2) * sub_stride16;
-                const uint32_t d = tmem_base + static_cast<uint32_t>(a2) * 256u;
-                for (int k = 0; k < ksteps; ++k)
-                  ptx::umma_f16_lohi(d, b_lo0 + 2 * k, x_lo + 2 * k, kDescHi, idesc, accumulate | static_cast<uint32_t>(k));
-              }
-              ptx::umma_commit(&emptyB[slotB]);
-            }
-          } else if (ptx::elect_one()) {
+          if (ptx::elect_one()) {
             for (int s = 0; s < nacc_eff; ++s) {
               const uint32_t a_lo = a_lo1 + static_cast<uint32_t>(s) * sub_stride16;
               const uint32_t d = tmem_base + static_cast<uint32_t>(s) * ncta;
@@ -529,81 +515,7 @@ __global__ void __launch_bounds__(kThreads, 1)
     const int chalf = p.up_time == 2 ? p.Cout / 2 : p.Cout;
     const int bias_b = (p.flags & CVVAE_CONV_W_PER_BATCH) ? 0 : tc.b;  // batched GEMM: a row bias is shared by the batch items
     int item = 0;
-    if (p.tma_epi && p.swap) {
-      // ---- swapped orientation: this thread owns output channel c = 32q + lane, a 32x32b TMEM load gives it 32
-      // consecutive positions.  Staging tile = [32 positions][32 channels] (64-byte rows, no swizzle): a warp's 16-bit
-      // stores of one position are 64 contiguous bytes (conflict-free); one TMA store per tile as in the other path.
-      uint8_t* stage = sA + static_cast<size_t>(warp) * 8192;
-      uint32_t res_phase = 0;
-      int nbuf = 0;
-      const int c_me = tc.n0 + q * 32 + lane;
-      const float bias_c = (p.bias && !(p.flags & CVVAE_CONV_BIAS_ALONG_M) && c_me < p.Cout) ? __ldg(p.bias + c_me) : 0.f;
-      float gs = 0.f, gq = 0.f;  // this channel's GroupNorm partial sums over all items of the CTA
-      for (int a2 = 0; 2 * a2 < nacc_eff; ++a2) {
-        for (int j = 0; j < 8; ++j) {
-          const int f0 = a2 * 256 + j * 32;           // first flattened tile position of this item
-          if (f0 >= nacc_eff * 128) break;             // warp-uniform
-          if (((item++) & 1) != grp) continue;         // warp-uniform
-          const int h = tc.h0 + f0 / p.TW, w = tc.w0 + f0 % p.TW;
-          // validity of the 32 positions (lane i <-> position i), shared through a ballot
-          const int hi = tc.h0 + (f0 + lane) / p.TW, wi = tc.w0 + (f0 + lane) % p.TW;
-          const unsigned valid = __ballot_sync(0xffffffffu, (hi < p.H_out) && (wi < p.W_out));
-          uint8_t* tile = stage + (nbuf & 1) * 2048;
-          const uint32_t tile_u32 = ptx::smem_u32(tile);
-          if (lane == 0) ptx::bulk_wait_read<1>();
-          __syncwarp();
-          if (p.residual) {
-            if (lane == 0) {
-              ptx::mbar_expect_tx(&resBar[warp], 2048);
-              ptx::tma_load_5d(tile, &tmR, &resBar[warp], tc.n0 + q * 32, w, h, tc.t, tc.b);
-            }
-            wait_bar(&resBar[warp], res_phase);
-            res_phase ^= 1;
-          }
-          uint32_t v[32];
-          ptx::tmem_ld_32x32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(a2 * 256 + j * 32), v);
-          ptx::tmem_ld_wait();
-          const uint32_t my = tile_u32 + static_cast<uint32_t>(lane) * 2u;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            float a = fmaf(__uint_as_float(v[i]), p.alpha, bias_c);
-            if (p.residual) {
-              uint16_t r16;
-              asm volatile("ld.shared.u16 %0, [%1];" : "=h"(r16) : "r"(my + i * 64u));
-              a += E::to_f(*reinterpret_cast<const typename E::T*>(&r16));
-            }
-            const typename E::T o = E::from_f(a);
-            if (p.gn_stats && ((valid >> i) & 1u)) {
-              const float of = E::to_f(o);
-              gs += of;
-              gq = fmaf(of, of, gq);
-            }
-            asm volatile("st.shared.u16 [%0], %1;" ::"r"(my + i * 64u), "h"(*reinterpret_cast<const uint16_t*>(&o)) : "memory");
-          }
-          ptx::fence_proxy_async();
-          __syncwarp();
-          if (lane == 0) {
-            ptx::tma_store_5d(&tmY, tile, tc.n0 + q * 32, w, h, tc.t, tc.b);
-            ptx::bulk_commit();
-          }
-          ++nbuf;
-        }
-      }
-      if (p.gn_stats) {
-        // channels of one group are neighbouring lanes: reduce over cpg lanes, the first lane of each group adds
-        for (int o = 1; o < p.gn_cpg && o < 32; o <<= 1) {
-          gs += __shfl_xor_sync(0xffffffffu, gs, o);
-          gq += __shfl_xor_sync(0xffffffffu, gq, o);
-        }
-        const int lanes_per_group = min(p.gn_cpg, 32);
-        if ((lane % lanes_per_group) == 0 && c_me < p.yC) {
-          atomicAdd(&gn_bins[(c_me / p.gn_cpg) * 2], gn_fix(gs, kGnSumScale));
-          atomicAdd(&gn_bins[(c_me / p.gn_cpg) * 2 + 1], gn_fix(gq, kGnSqScale));
-        }
-      }
-      if (lane == 0) ptx::bulk_wait<0>();
-      __syncwarp();
-    } else if (p.tma_epi) {
+    if (p.tma_epi) {
       // ---- TMEM -> registers -> SWIZZLE_128B staging tile (32 positions x 64 channels, 4 KB) -> TMA store.
       // A warp's direct 16-byte stores would touch 32 different 128-byte lines per instruction (position stride
       // = C*2 bytes); the bulk tensor store writes full lines and clips partial tiles by itself.  The residual
@@ -1332,25 +1244,6 @@ static bool encode_map(CUtensorMap* m, const void* ptr, int rank, const cuuint64
   return true;
 }
 
-// Experiment knobs (environment), read ONCE per process - nothing on the launch path calls getenv.
-struct Knobs {
-  int nacc, persist, fill, cta_group, tw, na, swap, wide, wide2, pw, smem_reserve;
-  static int env(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-  }
-  Knobs()
-      : nacc(env("CVVAE_CONV_NACC", 0)), persist(env("CVVAE_CONV_PERSIST", 1)), fill(env("CVVAE_CONV_FILL", 1)),
-        cta_group(env("CVVAE_CONV_CTA_GROUP", 0)), tw(env("CVVAE_CONV_TW", 0)), na(env("CVVAE_CONV_NA", 0)),
-        swap(env("CVVAE_CONV_SWAP", 1)), wide(env("CVVAE_CONV_WIDE", 1)), wide2(env("CVVAE_CONV_WIDE2", 1)),
-        pw(env("CVVAE_CONV_PW", 0)),
-        smem_reserve(env("CVVAE_CONV_SMEM_RESERVE", 0)) {}
-};
-static const Knobs& knobs() {
-  static const Knobs k;
-  return k;
-}
-
 bool conv_tc_eligible(const cvvae_conv_desc* d, const char** why) {
   const cvvae_tensor5& x = d->x;
   auto fail = [&](const char* m) {
@@ -1440,27 +1333,18 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
   p.N_cta = N_cta;
   p.n_tiles_n = (p.Cout + N_cta - 1) / N_cta;
   p.NACC = (512 / N_cta) < 4 ? (512 / N_cta) : 4;
-  const Knobs& kn = knobs();
-  // experiment knob: fewer accumulators per CTA (halves the reuse of each staged weight tile)
-  if (kn.nacc > 0 && kn.nacc < p.NACC) p.NACC = kn.nacc;
-  // persistent double-buffered variant for the Cout == 128 layers: tiles of 256 positions (two 128-row sub-tiles)
-  const int persist_env = kn.persist;
-  const bool flat_shape = (p.H_out == 1 && d->KH == 1 && d->KW == 1 && d->sw == 1 && d->sh == 1 && x.H == 1);
-  const bool persist_want = persist_env && !flat_shape && p.Cout == 128 && N_cta == 128 && p.up_time == 1 && p.vec_ok &&
-                            !(d->flags & (CVVAE_CONV_BIAS_ALONG_M | CVVAE_CONV_OUT_F32)) && y.C % 32 == 0;
-  if (persist_want) p.NACC = 2;
-  // wide slabs (one slab per (kt, channel block) for all KH x KW taps): stride-1 spatial kernels of the persistent path
-  const bool wide_want = persist_want && kn.wide && kn.swap && kn.cta_group != 2 && kn.nacc == 0 && d->sh == 1 && d->sw == 1 &&
-                         d->KW > 1 && d->KW <= 3 && d->KH <= 3;
-  // ... and of the Cout >= 256 layers (non-persistent kernel, CTA pairs side by side along W)
-  const bool wide2_want = !persist_want && kn.wide2 && N_cta == 256 && kn.nacc == 0 && kn.tw == 0 && d->sh == 1 && d->sw == 1 &&
-                          d->KW > 1 && d->KW <= 3 && d->KH <= 3 && !flat_shape;
-  const bool wide_any = wide_want || wide2_want;
   p.flat = (p.H_out == 1 && d->KH == 1 && d->KW == 1 && d->sw == 1 && d->sh == 1 && x.H == 1) ? 1 : 0;
   if (d->flags & (CVVAE_CONV_W_PER_BATCH | CVVAE_CONV_X_SHARED))
     CVVAE_CHECK_ARG(p.flat, "conv: batched-GEMM flags need a flat problem (H == 1, 1x1x1, stride 1)");
+  // persistent double-buffered kernel for the Cout == 128 layers: tiles of 256 positions (two 128-row sub-tiles)
+  p.persist = (!p.flat && p.Cout == 128 && p.up_time == 1 && p.vec_ok &&
+               !(d->flags & (CVVAE_CONV_BIAS_ALONG_M | CVVAE_CONV_OUT_F32)) && y.C % 32 == 0) ? 1 : 0;
+  if (p.persist) p.NACC = 2;
+  // wide slabs (one slab per (kt, channel block) for all KH x KW taps) for stride-1 spatial kernels, in the persistent
+  // kernel and in the Cout >= 256 layers (non-persistent kernel, CTA pairs side by side along W)
+  const bool wide_want = (p.persist || N_cta == 256) && !p.flat && d->sh == 1 && d->sw == 1 && d->KW > 1 && d->KW <= 3 &&
+                         d->KH <= 3;
   p.cblocks = (p.Cin + 63) / 64;
-  const int fill_env = kn.fill;   // experiment knob: 0 keeps the widest tiles even when they leave SMs idle
   for (;;) {
   if (p.flat) {
     p.TW = 128; p.ROWS = 1; p.TH = 1;
@@ -1472,8 +1356,8 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
     p.n_hgroups = d->KH / p.KHs;
     long long best_cost = -1;
     int best_tw = 16;
-    // CTA pairs stack two tiles vertically: an odd tile count costs one whole padding tile per column of tiles
-    const int cg_plan = kn.cta_group == 1 ? 1 : ((kn.cta_group == 2 || N_cta == 256) ? 2 : 1);
+    // CTA pairs (N_cta = 256) stack two tiles vertically: an odd tile count costs one whole padding tile per column of tiles
+    const int cg_plan = N_cta == 256 ? 2 : 1;
     for (int tw = 8; tw <= 128; tw *= 2) {
       const int rows = 128 / tw;
       const int th = rows * p.NACC;
@@ -1492,11 +1376,7 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
         best_tw = tw;
       }
     }
-    const int tw_env = kn.tw;   // experiment knob: force the tile width
-    if (tw_env >= 8 && tw_env <= 128 && (tw_env & (tw_env - 1)) == 0 && tw_env * d->sw <= 256 &&
-        ((128 / tw_env) * p.NACC + p.KHs - 1) * d->sh <= 256)
-      best_tw = tw_env;
-    if (wide_any) best_tw = 8;   // one 8-row swizzle group per image row of the tile
+    if (wide_want) best_tw = 8;   // one 8-row swizzle group per image row of the tile
     p.TW = best_tw;
     p.ROWS = 128 / p.TW;
     p.TH = p.ROWS * p.NACC;
@@ -1507,50 +1387,46 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
   // small problems (latent-resolution layers, single images, attention GEMMs): fewer accumulators per CTA = more CTAs.
   // The count is per SAMPLE so that the plan - hence every rounding - is independent of the batch size.
   const long long ctas_per_sample = 1ll * p.n_tiles_n * p.T_out * p.tiles_w * p.tiles_h;
-  if (!fill_env || persist_want || p.NACC <= 1 || ctas_per_sample >= num_sms()) break;
+  if (p.persist || p.NACC <= 1 || ctas_per_sample >= num_sms()) break;
   p.NACC /= 2;
   }
   p.slab_bytes = p.flat ? static_cast<uint32_t>(p.NACC) * 16384u : static_cast<uint32_t>(p.slab_rows * p.TW) * 128u;
   p.wide = 0;
   p.PW = p.TW;
-  if (wide_any && !p.flat) {
+  if (wide_want) {
     p.wide = 1;
     p.PW = 8 + d->KW - 1;
-    if (kn.pw > p.PW && kn.pw <= 32) p.PW = kn.pw;   // experiment knob: slab pitch in positions
     p.slab_bytes = static_cast<uint32_t>(p.slab_rows * p.PW) * 128u;
   }
   p.slab_stride = (p.slab_bytes + 1023u) & ~1023u;
-  // CTA pairs (cta_group::2) when there are at least two vertically adjacent tiles to pair up
-  const int cg_env = kn.cta_group;
-  // measured (tools/bench_conv.py): pairs help the N_cta = 256 layers (half the weight bytes per CTA, up to +10 %)
-  // and cost 0-16 % on the N_cta = 128 layers, so they are on for N_cta = 256 only (CVVAE_CONV_CTA_GROUP=2 forces them
-  // wherever possible, =1 switches them off)
-  p.pair_w = (p.wide && !persist_want) ? 1 : 0;   // wide slabs: 8-wide tiles, pair them along W (always plenty, never odd rows)
-  const bool pair_ok = !p.flat && (p.pair_w ? p.tiles_w >= 2 : p.tiles_h >= 2) && N_cta >= 32;
-  const int CG = (cg_env == 1 || !pair_ok) ? 1 : ((cg_env == 2 || N_cta == 256) ? 2 : 1);
+  // CTA pairs (cta_group::2) when there are at least two adjacent tiles to pair up.  Measured (tools/bench_conv.py): pairs
+  // help the N_cta = 256 layers (half the weight bytes per CTA, up to +10 %) and cost 0-16 % on the N_cta = 128 layers,
+  // so they are used for N_cta = 256 only
+  p.pair_w = (p.wide && !p.persist) ? 1 : 0;   // wide slabs: 8-wide tiles, pair them along W (always plenty, never odd rows)
+  const bool pair_ok = !p.flat && (p.pair_w ? p.tiles_w >= 2 : p.tiles_h >= 2);
+  const int CG = (pair_ok && N_cta == 256) ? 2 : 1;
   p.tiles_hg = p.pair_w ? p.tiles_h : (p.tiles_h + CG - 1) / CG;
   p.tiles_wg = p.pair_w ? (p.tiles_w + CG - 1) / CG : p.tiles_w;
   p.b_bytes = static_cast<uint32_t>(N_cta / CG) * 128u;  // weight rows staged per CTA
-  p.idesc = ptx::umma_idesc_f16(d->dtype == CVVAE_BF16 ? 1 : 0, 128 * CG, N_cta);
+  // the persistent kernel swaps the MMA operands: D = [128 channels][256 positions]
+  p.idesc = p.persist ? ptx::umma_idesc_f16(d->dtype == CVVAE_BF16 ? 1 : 0, 128, 256)
+                      : ptx::umma_idesc_f16(d->dtype == CVVAE_BF16 ? 1 : 0, 128 * CG, N_cta);
 
   // ---- shared memory budget: 227 KB - alignment slack - barriers
-  // (CVVAE_CONV_SMEM_RESERVE leaves shared memory free for CTAs of a memory-bound kernel from another stream to co-reside)
-  const size_t reserve = kn.smem_reserve > 0 && kn.smem_reserve <= 32768 ? static_cast<size_t>(kn.smem_reserve) : 0;
-  const size_t budget = 232448 - 1024 - 1536 - (persist_want ? 32768 : 0) - reserve;  // persistent kernel: own staging area
+  const size_t budget = 232448 - 1024 - 1536 - (p.persist ? 32768 : 0);  // persistent kernel: own staging area
   int NB = 4;
   while (NB > 2 && static_cast<size_t>(NB) * p.b_bytes + 2ull * p.slab_stride > budget) --NB;
   size_t rest = budget - static_cast<size_t>(NB) * p.b_bytes;
   int NA = static_cast<int>(rest / p.slab_stride);
   if (p.wide && NA > 2) NA = 2;   // a wide slab lasts KH x KW weight tiles: two slots hide its load, the rest goes to weights
   if (NA > 4) NA = 4;
-  if (kn.na >= 2 && kn.na < NA) NA = kn.na;   // experiment knob: cap the slab ring (the rest goes to weight slots)
   CVVAE_CHECK_ARG(NA >= 2, "conv_tc: slab of %u bytes does not fit the shared-memory budget", p.slab_bytes);
   // spend what is left on more weight stages
   while (NB < 8 && static_cast<size_t>(NB + 1) * p.b_bytes + static_cast<size_t>(NA) * p.slab_stride <= budget) ++NB;
   p.NA = NA;
   p.NB = NB;
   const size_t smem = 1024 + static_cast<size_t>(NA) * p.slab_stride + static_cast<size_t>(NB) * p.b_bytes + 1536 +
-                      (persist_want ? 32768 : 0);
+                      (p.persist ? 32768 : 0);
 
   // ---- tensor maps
   CUtensorMap tmA, tmB;
@@ -1616,7 +1492,8 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
     }
   }
 
-  // ---- epilogue through shared memory + TMA store where the output is a plain channels-last 16-bit tensor
+  // ---- epilogue through shared memory + TMA store where the output is a plain channels-last 16-bit tensor.  The
+  // persistent kernel's transposing epilogue stages [32 positions][32 channels] tiles (64-byte rows, no swizzle).
   CUtensorMap tmY = tmA, tmR = tmA;
   p.tma_epi = 0;
   {
@@ -1629,23 +1506,16 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
       cuuint64_t strides[4] = {(cuuint64_t)y.s_w * 2, (cuuint64_t)y.s_h * 2, (cuuint64_t)y.s_t * 2, (cuuint64_t)y.s_b * 2};
       for (int i = 0; i < 4; ++i)
         if (dims[i + 1] == 1 && (strides[i] == 0 || strides[i] % 16)) strides[i] = (cuuint64_t)y.C * 2;
-      cuuint32_t box[5] = {64, (cuuint32_t)p.box_w, (cuuint32_t)(32 / p.box_w), 1, 1}, estr[5] = {1, 1, 1, 1, 1};
-      if (!encode_map(&tmY, y.ptr, 5, dims, strides, box, estr)) return CVVAE_E_CUDA;
-      if (d->residual && !encode_map(&tmR, d->residual, 5, dims, strides, box, estr)) return CVVAE_E_CUDA;
+      cuuint32_t box[5] = {p.persist ? 32u : 64u, (cuuint32_t)p.box_w, (cuuint32_t)(32 / p.box_w), 1, 1}, estr[5] = {1, 1, 1, 1, 1};
+      const CUtensorMapSwizzle swz = p.persist ? CU_TENSOR_MAP_SWIZZLE_NONE : CU_TENSOR_MAP_SWIZZLE_128B;
+      if (!encode_map(&tmY, y.ptr, 5, dims, strides, box, estr, swz)) return CVVAE_E_CUDA;
+      if (d->residual && !encode_map(&tmR, d->residual, 5, dims, strides, box, estr, swz)) return CVVAE_E_CUDA;
       p.tma_epi = 1;
-      // Cout == 128 layers: swap the MMA operands (see the issue loop) - needs the TMA epilogue's transposing stage
-      const int swap_env = kn.swap;
-      p.swap = (swap_env && !p.flat && CG == 1 && p.Cout == 128 && N_cta == 128 && (p.NACC == 4 || p.NACC == 2) && p.up_time == 1 &&
-                !(d->flags & CVVAE_CONV_BIAS_ALONG_M)) ? 1 : 0;
-      if (p.swap) {
-        cuuint32_t box2[5] = {32, (cuuint32_t)p.box_w, (cuuint32_t)(32 / p.box_w), 1, 1};
-        if (!encode_map(&tmY, y.ptr, 5, dims, strides, box2, estr, CU_TENSOR_MAP_SWIZZLE_NONE)) return CVVAE_E_CUDA;
-        if (d->residual && !encode_map(&tmR, d->residual, 5, dims, strides, box2, estr, CU_TENSOR_MAP_SWIZZLE_NONE)) return CVVAE_E_CUDA;
-        p.idesc = ptx::umma_idesc_f16(d->dtype == CVVAE_BF16 ? 1 : 0, 128, 256);
-        p.persist = (persist_want && p.NACC == 2) ? 1 : 0;
-      }
     }
   }
+  // a persistent plan always qualifies: its output is 16-byte aligned channels-last, and its slabs hold at least
+  // 256 positions x 128 B with NA >= 2
+  CVVAE_CHECK_ARG(!p.persist || p.tma_epi, "conv_tc: internal: persistent plan without the TMA epilogue");
   // fused GroupNorm statistics need the TMA epilogue, power-of-two channels per group and one sample per CTA index
   p.gn_stats = nullptr;
   if (d->gn_stats) {
@@ -1662,10 +1532,8 @@ int conv_tc_launch(const cvvae_conv_desc* d, cudaStream_t stream) {
     p.gn_cpg = cpg;
   }
 
-  CVVAE_CHECK_ARG(!wide_want || !p.wide || p.persist, "conv_tc: internal: wide-slab plan without the persistent kernel");
-  if (p.cblocks2 && ((p.swap && !p.persist) || (p.persist && !p.wide))) {
-    // (neither arises with the default knobs: stride-1 spatial kernels with Cout == 128 take the wide persistent path)
-    set_error("conv_tc: fused shortcut unsupported on the operand-swapped paths without wide slabs");
+  if (p.cblocks2 && p.persist && !p.wide) {
+    set_error("conv_tc: fused shortcut unsupported on the persistent kernel without wide slabs");
     return CVVAE_E_UNSUPPORTED;
   }
   const long long grid = 1ll * p.n_tiles_n * p.T_out * p.tiles_wg * p.tiles_hg * p.B * CG;

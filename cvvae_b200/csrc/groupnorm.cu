@@ -5,8 +5,6 @@
 // Replaces Normalize()+nonlinearity (reference models/vae_models.py:187-195,392-401), nn.GroupNorm+nn.SiLU
 // of models/vae_blocks3d_sd3.py, and norm_t (models/vae_models.py:571).  One rounding to 16 bit at the
 // end instead of the reference's three (GN out, sigmoid, product).
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace cvvae {
@@ -374,22 +372,6 @@ extern "C" int cvvae_groupnorm_apply(const cvvae_tensor5* x, const cvvae_tensor5
   const int units = per_frame ? x->B * x->T : x->B;
   dim3 grid;
   pick_grid(v, units, grid);
-  {
-    // experiment knob: cap the apply grid at this many CTAs per SM (grid-stride over the positions; no reduction in this
-    // kernel, so the split changes no bits) - lets the pass co-reside with a tensor-bound kernel of another stream
-    static const int cap = [] {
-      const char* e = getenv("CVVAE_GN_CTAS_PER_SM");
-      return e ? atoi(e) : 0;
-    }();
-    if (cap > 0) {
-      long long per_unit = (1ll * cap * num_sms() + units - 1) / units;
-      if (per_unit < 1) per_unit = 1;
-      long long ppb = (v.pix_per_unit + per_unit - 1) / per_unit;
-      if (ppb < 256) ppb = 256;
-      v.pix_per_block = ppb;
-      grid = dim3(static_cast<unsigned>((v.pix_per_unit + ppb - 1) / ppb), static_cast<unsigned>(units));
-    }
-  }
   const size_t smem = sizeof(float) * 2 * x->C;
   const long long* st = reinterpret_cast<const long long*>(stats);
   // 4 loads in flight per thread + streaming (no-allocate / evict-first) accesses: 5.7 TB/s on 1.4 GB tensors, 87 % of the

@@ -18,7 +18,6 @@ All arithmetic goes through an ``ops`` backend (``cvvae_b200.ops.CudaOps`` in pr
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import Dict, Optional, Tuple
 
@@ -130,9 +129,8 @@ class Engine:
         self._stats_arena = None   # [slots, B, groups, 2] int64, zeroed once per network pass
         self._stats_next = 0
         self.attn_scratch_bytes = 4 << 30  # cap of the fp32 logits buffer of the batched spatial attention
-        # 1x1 shortcuts as extra K steps of conv2 (CVVAE_FUSE_SHORTCUT=0: separate launch + residual add, for A/B runs)
-        # (the experiment knob CVVAE_CONV_WIDE=0 selects a persistent-kernel variant without the shortcut K steps)
-        self.fuse_shortcut = os.environ.get("CVVAE_FUSE_SHORTCUT", "1") != "0" and os.environ.get("CVVAE_CONV_WIDE", "1") != "0"
+        # 1x1 shortcuts run as extra K steps of conv2 (resblock); inputs _tc_ok rejects take a separate launch + residual add
+        self.fuse_shortcut = True
 
     # ------------------------------------------------------------------ shape arithmetic
     def encoded_frames(self, T: int) -> int:

@@ -115,7 +115,9 @@ CONV_CASES = {
                     {"lattice_out": (0, 1)}),
     "phase322": ((1, 2, 20, 16, 128), 256, (3, 2, 2), (1, 1, 1), ((1, 1), (0, 1), (1, 0)), PAD_REPLICATE, PAD_ZERO, 1,
                  {"lattice_out": (1, 0)}),
-    # tall enough for CTA pairs (cta_group::2): even / odd number of row tiles, strided, interleaved, residual
+    # tall problems: pair_n256_odd / pair_n512 / pair_phase_up take CTA pairs (cta_group::2) along W with an odd tile count
+    # (residual, interleaved); pair_n128 the persistent wide-slab kernel, pair_down the persistent kernel without wide slabs
+    # (strided), pair_cout32 the single-CTA kernel.  Pairs along H: conv1x1_spatial
     "pair_n128": ((1, 3, 80, 48, 64), 128, (3, 3, 3), (1, 1, 1), ((2, 0), (1, 1), (1, 1)), PAD_REPLICATE, PAD_ZERO, 1, {}),
     "pair_n256_odd": ((1, 2, 72, 40, 128), 256, (3, 3, 3), (1, 1, 1), ((1, 1), (1, 1), (1, 1)), PAD_ZERO, PAD_ZERO, 1,
                       {"residual": True}),
@@ -329,18 +331,6 @@ def test_conv_fused_groupnorm_stats(name):
     # outputs may differ by one fp16 rounding flip (2^-10 relative) on a few elements - inside the contract
     _assert_close(ops.groupnorm(y, g, b, 32, 1e-5, stats=stats).float(), ops.groupnorm(y, g, b, 32, 1e-5).float(), 1e-3, 1e-4,
                   f"gn_fused_stats_{name}")
-
-
-def test_conv_pairs_forced_everywhere():
-    """CTA pairs are enabled by default only where they pay (N_cta = 256); re-run the conv cases with
-    CVVAE_CONV_CTA_GROUP=2 (pairs wherever two row tiles exist) in a fresh process."""
-    import subprocess
-    import sys
-    env = dict(os.environ, CVVAE_CONV_CTA_GROUP="2")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-m", "gpu", "-k",
-                        "test_conv_tc_matches_spec or test_conv_fused_groupnorm_stats"], env=env, capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-1000:]
 
 
 @pytest.mark.parametrize("shape,cout,kt,off_t,pad_t", [((1, 3, 40, 50, 128), 3, 3, -1, PAD_ZERO), ((2, 5, 33, 61, 128), 3, 3, -2, PAD_REPLICATE),
